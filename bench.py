@@ -30,6 +30,7 @@ CRITEO_1TB_40M = [39884406, 39043, 17289, 7420, 20263, 3, 7120, 1543, 63, 385329
                   39979771, 25641295, 39664984, 585935, 12972, 108, 36]
 HOST_HEAD_STEPS = 16  # host enqueue time is averaged over this many steps right after the start barrier
 BASELINE_SAMPLES_PER_SEC = {1: 50_000.0, 8: 350_000.0}  # reference published numbers (A100), BASELINE.md
+DUMP_BYTES = 64 << 20  # --dump-outputs budget over all ranks
 
 
 def parse_args() -> argparse.Namespace:
@@ -67,6 +68,9 @@ def parse_args() -> argparse.Namespace:
     p.add_argument("--phase-times", action="store_true", help="diagnostics: forward / backward / optimizer device time of the plain step (stderr)")
     p.add_argument("--trace-e2e", type=str, default="", help="diagnostics: torch.profiler trace (chrome json + op table) of 6 extra pipeline steps")
     p.add_argument("--num-host-batches", type=int, default=8)
+    p.add_argument("--dump-outputs", type=str, default="", metavar="DIR",
+                   help="write what the last timed step returned (loss, logits, labels) as DIR/<name>.npy in float32, to compare two builds "
+                        "output for output; with several GPUs each rank writes <name>_rank<r>.npy")
     return p.parse_args()
 
 
@@ -375,6 +379,24 @@ def fp8_inference_qps(args, dmp, device, rank: int, world: int, keys, hashes) ->
             "l2_policy": "16 distinct one-hot batches (1.9 GB of rows) cycled: no batch is served from the 126 MB L2", "out_shape": list(out.shape)}
 
 
+def dump_outputs(directory: str, arrays: Dict[str, Any], rank: int, world: int) -> None:
+    """Writes one step's outputs as float32 ``<name>.npy`` files. All ranks together write at most DUMP_BYTES: when the per-sample
+    arrays are longer than this rank's share, the same fixed, seeded sample of samples is kept from every array."""
+    import numpy as np
+    import torch
+
+    host = {k: v.detach().float().reshape(-1).cpu() for k, v in arrays.items()}
+    n = max(t.numel() for t in host.values())
+    cap = DUMP_BYTES // (4 * len(host) * world)
+    if n > cap:
+        keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:cap].sort().values
+        host = {k: t[keep] if t.numel() == n else t for k, t in host.items()}
+    os.makedirs(directory, exist_ok=True)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    for k, t in host.items():
+        np.save(os.path.join(directory, f"{k}{suffix}.npy"), t.numpy())
+
+
 def main() -> None:
     args = parse_args()
     if args.impl == "reference":
@@ -411,6 +433,7 @@ def main() -> None:
         os.environ["TRB_TRANSPORT"] = args.transport  # "nccl": the internal UNFUSED arm (own lookup kernels + NCCL all-to-alls)
     _lib.lib()
 
+    torch.manual_seed(0)  # model initialisation, like the batches below, is the same in every run with the same arguments
     dmp, opt, keys, hashes, ids_per_feature, num_dense, dense_backend, plan_info = build_ours(args, device, rank, world)
     B = args.batch_size
     ds = RandomRecDataset(keys, B, hash_sizes=hashes, ids_per_features=ids_per_feature, num_dense=num_dense, manual_seed=1234 + rank,
@@ -437,12 +460,12 @@ def main() -> None:
         args.cuda_graphs = 0
         dmp.init_data_parallel()
 
-    def step(batch) -> "torch.Tensor":
+    def step(batch):
         opt.zero_grad()
-        loss, _ = dmp(batch)
+        loss, out = dmp(batch)
         loss.backward()
         opt.step()
-        return loss
+        return loss, out
 
     def barrier() -> None:
         if world > 1:
@@ -463,7 +486,7 @@ def main() -> None:
     t_host0 = time.perf_counter()
     t_host_head = None
     for i in range(args.steps):
-        loss = step(dev_batches[i % len(dev_batches)])
+        loss, out = step(dev_batches[i % len(dev_batches)])
         if i == HOST_HEAD_STEPS - 1:
             t_host_head = time.perf_counter()
     # CPU time to ENQUEUE a step (>= ms_per_step means launch-bound). Measured over the first steps after the barrier: once the host
@@ -473,6 +496,8 @@ def main() -> None:
     barrier()
     ms = e0.elapsed_time(e1)
     launches = _lib.launch_count() - n0
+    if args.dump_outputs:  # before any further step: with CUDA graphs the logits live in a buffer the next replay overwrites
+        dump_outputs(args.dump_outputs, {"loss": loss, "logits": out[1], "labels": out[2]}, rank, world)
     if args.phase_times:  # diagnostics: where the device time of the plain step goes (events on the main stream, no profiler attached)
         n_ph = 20
         evs = [[torch.cuda.Event(enable_timing=True) for _ in range(4)] for _ in range(n_ph)]
